@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the rasteriser hot path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl b200|reference]
+    python bench.py --gpus N --steps K --warmup W [--impl b200|reference] [--dump-outputs DIR]
     (N > 1: launched by torch.distributed.run, one rank per GPU)
 
 A "step" is one pass of the hot path over one view: forward (GaussianPointCloudRasterisation,
@@ -57,7 +57,11 @@ def parse_args():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=WORKLOAD)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--repeats", type=int, default=10, help="extra timed regions of --steps steps each (median / p10 / p90)")
+    ap.add_argument("--repeats", type=int, default=0,
+                    help="extra timed regions of --steps steps each after the first; the headline is the median region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32): image, "
+                         "depth, valid point count and the gradient rows of a fixed, seeded sample of Gaussians")
     ap.add_argument("--exchange-streams", type=int, default=1, choices=[1, 2],
                     help="N > 1: 2 = the all-gather of the compact exchange on a second NCCL communicator, concurrent with the all-reduce")
     ap.add_argument("--exchange", default="auto", choices=["auto", "multimem", "nccl"],
@@ -145,8 +149,8 @@ def oracle_step(scene, band=3):
     from helpers import oracle_backward, oracle_forward
     o, fwd, feats = oracle_forward(scene)
     g = np.ones(fwd.image.shape, np.float32)
-    oracle_backward(o, fwd, scene, feats, g, band)
-    return fwd
+    bwd = oracle_backward(o, fwd, scene, feats, g, band)
+    return fwd, bwd
 
 
 def pin_cpu_threads():
@@ -182,8 +186,12 @@ def run_reference(args):
     per_step = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        oracle_step(scene)
+        fwd, bwd = oracle_step(scene)
         per_step.append((time.perf_counter() - t0) * 1e3)
+    if args.dump_outputs:
+        import torch
+        dump_outputs(args.dump_outputs, *(torch.from_numpy(a) for a in (
+            fwd.image, fwd.depth, fwd.pixel_valid_point_count, bwd.grad_pointcloud, bwd.grad_pointcloud_features)))
     dt = sum(per_step) / 1e3
     value = H * W * args.steps / dt / 1e6
     cores = gs_oracle.num_threads()
@@ -210,6 +218,24 @@ FP32_LANE_PEAK = NUM_SMS * 128 * SM_CLOCK_HZ    # FP32 lane operations / s (an F
 MUFU_LANE_PEAK = NUM_SMS * 16 * SM_CLOCK_HZ     # MUFU (ex2 / rcp) lane operations / s
 # SASS instructions per (warp, splat) visit of the inner loops (cuobjdump of this build, DESIGN section 3)
 FWD_INSTR_PER_VISIT, BWD_INSTR_PER_VISIT = 29, 30 + 34
+DUMP_BYTES = 60_000_000  # array data of --dump-outputs: the files stay under 64 MB with their headers
+
+
+def dump_outputs(out_dir, image, depth, count, grad_xyz, grad_features):
+    """Write one step's outputs as float32 .npy files so that two builds can be compared output for output.  The per-pixel
+    outputs are written whole; the dense gradients of 1e6 Gaussians (236 MB) do not fit the budget, so the rows of a fixed,
+    seeded sample of Gaussians (the same for the same workload) fill what the pixels leave of it."""
+    import numpy as np
+    import torch
+    pixel_bytes = 4 * (image.numel() + depth.numel() + count.numel())
+    n = grad_xyz.shape[0]
+    num_rows = min(n, (DUMP_BYTES - pixel_bytes) // (4 * (grad_xyz.shape[1] + grad_features.shape[1])))
+    rows = np.sort(np.random.default_rng(0).choice(n, num_rows, replace=False))
+    idx = torch.from_numpy(rows).to(grad_xyz.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("image", image), ("depth", depth), ("pixel_valid_point_count", count),
+                    ("grad_pointcloud_sampled_rows", grad_xyz[idx]), ("grad_pointcloud_features_sampled_rows", grad_features[idx])):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to(torch.float32).cpu().numpy())
 
 
 def run_b200(args):
@@ -312,8 +338,8 @@ def run_b200(args):
             sc = self.scene
             sc.point_cloud.grad = None
             sc.point_cloud_features.grad = None
-            image, _, _ = self.op(self.dev_input)
-            image.backward(self.grad_image)  # N > 1: the gradient exchange over NVLink happens inside this backward
+            self.outputs = self.op(self.dev_input)  # (image, depth, valid point count): kept for --dump-outputs
+            self.outputs[0].backward(self.grad_image)  # N > 1: the gradient exchange over NVLink happens inside this backward
             self.finish_step()
 
         def mpix(self, ms_per_step):
@@ -322,16 +348,18 @@ def run_b200(args):
     wl = Workload(args.workload)
     H, W, N, cfg, op, scene = wl.H, wl.W, wl.N, wl.cfg, wl.op, wl.scene
 
-    # ---- headline: inputs resident in HBM; EXACTLY `steps` steps in one timed region (the contract), then `repeats`
-    #      more regions of the same length for the spread
+    # ---- headline: inputs resident in HBM; one timed region of exactly `steps` steps, then `repeats` (default 0) more
+    #      regions of the same length
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
     for _ in range(warmup):
         wl.step()
-    # 1 + `repeats` timed regions of EXACTLY `steps` steps each; the headline is the MEDIAN region (BASELINE.md's protocol:
-    # median with p10 / p90 beside it), the first region is reported as well
+    # the headline is the MEDIAN region (BASELINE.md's protocol: median with p10 / p90 beside it, which takes --repeats), the
+    # first region is reported as well.  No event between the steps: one after every step costs 3-5 us per step (B200, 1000 W).
     regions = [timed(wl.step, steps) / steps for _ in range(1 + max(args.repeats, 0))]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *wl.outputs, scene.point_cloud.grad, scene.point_cloud_features.grad)
     first_region_ms = regions[0]
     ms_per_step = statistics.median(regions)
     value = wl.mpix(ms_per_step)

@@ -138,49 +138,73 @@ def main():
         print("wrote", len(small), "arrays")
     if with_c2r:
         # 976 x 544 pixels, 3.7e4 points, 4.9e5 pairs: keep hashes of everything that must be bit-equal and samples of the rest
-        import hashlib
         pre = "C2R_reduced_config_2/"
         full = {k[len(pre):]: v for k, v in out.items() if k.startswith(pre)}
-        digest = lambda a: np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), dtype=np.uint8)  # noqa: E731
-        keep = {}
-        for key in ("hook_point_id_in_camera_list", "hook_num_overlap_tiles", "hook_num_affected_pixels", "count",
-                    "stage_point_in_camera_sort_key", "stage_point_offset_with_sort_key", "stage_tile_points_start",
-                    "stage_tile_points_end", "stage_pixel_offset_of_last_effective_point", "stage_point_uv",
-                    "stage_point_in_camera", "stage_point_uv_conic_and_rescale", "stage_point_alpha_after_activation",
-                    "stage_point_color", "stage_point_radii", "features_after_forward"):
-            keep["sha256_" + key] = digest(full[key])
-        rng = np.random.default_rng(0)
-        h, w = full["count"].shape
-        pix = rng.choice(h * w, 6000, replace=False)
-        keep["pixel_index"] = pix
-        for key in ("image", "depth", "count", "stage_pixel_accumulated_alpha"):
-            keep["pixel_" + key] = full[key].reshape(h * w, -1)[pix]
-        tiles = full["image"].reshape(h // 16, 16, w // 16, 16, 3).astype(np.float64).sum(axis=(1, 3))
-        keep["tile_image_sum"] = tiles.astype(np.float32)
-        m = full["hook_point_id_in_camera_list"].shape[0]
-        rows = np.sort(rng.choice(m, 1500, replace=False))
-        keep["point_rows"] = rows
-        for key in ("hook_grad_point_in_camera", "hook_grad_pointfeatures_in_camera", "hook_grad_viewspace",
-                    "hook_magnitude_grad_viewspace"):
-            keep["rows_" + key] = full[key][rows]
-            keep["l1_" + key] = np.array([np.abs(full[key].astype(np.float64)).sum()])
-        keep["sizes"] = np.array([m, full["stage_point_offset_with_sort_key"].shape[0], int(full["count"].max())])
+        keep = {"sha256_" + key: digest(full[key]) for key in (
+            "hook_point_id_in_camera_list", "hook_num_overlap_tiles", "hook_num_affected_pixels", "count",
+            "stage_point_in_camera_sort_key", "stage_point_offset_with_sort_key", "stage_tile_points_start",
+            "stage_tile_points_end", "stage_pixel_offset_of_last_effective_point", *PER_POINT_STAGE, "features_after_forward")}
+        keep.update(samples(full, 6000, 1500))
+        keep["sizes"] = np.array([full["hook_point_id_in_camera_list"].shape[0], full["stage_point_offset_with_sort_key"].shape[0],
+                                  int(full["count"].max())])
         np.savez_compressed(os.path.join(HERE, "reference_path_c2_reduced.npz"), **keep)
         print("wrote", len(keep), "arrays for the reduced BASELINE config 2")
     if with_c1:
-        # keep the file small: the dense gradients are stored for the in-frustum rows only (the hook tensors), the rest is
-        # checked to be zero here
-        c1 = {k: v for k, v in out.items() if k.startswith("C1_")}
-        ids = c1["C1_baseline_config_1/hook_point_id_in_camera_list"].astype(np.int64)
-        for key in ("grad_pointcloud", "grad_pointcloud_features"):
-            dense = c1.pop(f"C1_baseline_config_1/{key}")
-            rest = np.ones(dense.shape[0], dtype=bool)
-            rest[ids] = False
-            assert not dense[rest].any()
-        c1.pop("C1_baseline_config_1/features_after_forward")
-        c1.pop("C1_baseline_config_1/hook_magnitude_grad_viewspace_on_image")
-        np.savez_compressed(os.path.join(HERE, "reference_path_c1.npz"), **c1)
-        print("wrote", len(c1), "arrays for BASELINE config 1")
+        pre = "C1_baseline_config_1/"
+        full = {k[len(pre):]: v for k, v in out.items() if k.startswith(pre)}
+        np.savez_compressed(os.path.join(HERE, "reference_path_c1.npz"), **reduce_c1(full))
+        print("wrote the arrays for BASELINE config 1")
+
+
+PER_POINT_STAGE = ("stage_point_uv", "stage_point_in_camera", "stage_point_uv_conic_and_rescale",
+                   "stage_point_alpha_after_activation", "stage_point_color", "stage_point_radii")
+
+
+def digest(a):
+    import hashlib
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), dtype=np.uint8)
+
+
+def samples(full, num_pixels, num_rows):
+    """Seeded samples of the float outputs: pixels of image / depth / count / accumulated alpha, per-tile image sums, rows of
+    the hook gradients with each gradient's L1 norm over all rows."""
+    keep = {}
+    rng = np.random.default_rng(0)
+    h, w = full["count"].shape
+    pix = rng.choice(h * w, num_pixels, replace=False)
+    keep["pixel_index"] = pix
+    for key in ("image", "depth", "count", "stage_pixel_accumulated_alpha"):
+        keep["pixel_" + key] = full[key].reshape(h * w, -1)[pix]
+    tiles = full["image"].reshape(h // 16, 16, w // 16, 16, 3).astype(np.float64).sum(axis=(1, 3))
+    keep["tile_image_sum"] = tiles.astype(np.float32)
+    m = full["hook_point_id_in_camera_list"].shape[0]
+    rows = np.sort(rng.choice(m, num_rows, replace=False))
+    keep["point_rows"] = rows
+    for key in ("hook_grad_point_in_camera", "hook_grad_pointfeatures_in_camera", "hook_grad_viewspace",
+                "hook_magnitude_grad_viewspace"):
+        keep["rows_" + key] = full[key][rows]
+        keep["l1_" + key] = np.array([np.abs(full[key].astype(np.float64)).sum()])
+    return keep
+
+
+def reduce_c1(full):
+    """BASELINE config 1 (256 x 256, 9566 points in the frustum) within 1 MB: the integer outputs the GPU test compares with
+    a tolerance are stored whole, every other array that must be bit-equal as a SHA-256, and the floats as a quarter of the
+    pixels and of the in-frustum rows.  The dense gradients are zero outside the frustum (checked here) and equal the hook
+    tensors inside it, so they are not stored."""
+    ids = full["hook_point_id_in_camera_list"].astype(np.int64)
+    for key, hook in (("grad_pointcloud", "hook_grad_point_in_camera"),
+                      ("grad_pointcloud_features", "hook_grad_pointfeatures_in_camera")):
+        rest = np.ones(full[key].shape[0], dtype=bool)
+        rest[ids] = False
+        assert not full[key][rest].any() and np.array_equal(full[key][ids], full[hook])
+    keep = {key: full[key] for key in ("hook_point_id_in_camera_list", "hook_num_overlap_tiles", "hook_num_affected_pixels",
+                                       "count", "stage_tile_points_start", "stage_tile_points_end")}
+    keep.update({"sha256_" + key: digest(full[key]) for key in (
+        "stage_point_in_camera_sort_key", "stage_point_offset_with_sort_key", "stage_pixel_offset_of_last_effective_point",
+        *PER_POINT_STAGE)})
+    keep.update(samples(full, 16384, 2400))
+    return keep
 
 
 if __name__ == "__main__":

@@ -161,13 +161,42 @@ def test_cuda_operator_reproduces_the_reference_kernels(name, exact_exp):
 
 # ---------------------------------------------------------------- BASELINE config 1 through the reference's kernels
 # reference_path_c1.npz: the same generator, run with --with-c1 (5 minutes in the interpreter), on SURVEY 8(d) C1 =
-# BASELINE config 1 (1e4 Gaussians, 256 x 256, SH deg 0).  The dense gradients are stored for the in-frustum rows only
-# (= the hook tensors; the other rows were checked to be zero when the file was made).
+# BASELINE config 1 (1e4 Gaussians, 256 x 256, SH deg 0).  Stored within 1 MB: ids, tile counts, pixel counts and tile
+# ranges whole, every other array that must be bit-equal as a SHA-256, the floats as samples (a quarter of the pixels
+# and of the in-frustum rows) beside per-tile image sums and each hook gradient's L1 norm.  The dense gradients are the
+# hook tensors on the in-frustum rows and zero elsewhere (checked when the file was made).
+def _digest(a):
+    import hashlib
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), dtype=np.uint8)
+
+
+def _tile_sums(image):
+    h, w = image.shape[:2]
+    return image.reshape(h // 16, 16, w // 16, 16, 3).astype(np.float64).sum(axis=(1, 3))
+
+
+C1_PER_POINT_STAGE = ("point_uv", "point_in_camera", "point_uv_conic_and_rescale", "point_alpha_after_activation", "point_color",
+                      "point_radii")
+
+
 def _c1():
     from reference_path_scenes import baseline_config_1
     g = np.load(os.path.join(HERE, "golden", "reference_path_c1.npz"))
-    prefix = "C1_baseline_config_1/"
-    return baseline_config_1(), SimpleNamespace(**{k[len(prefix):]: g[k] for k in g.files})
+    return baseline_config_1(), SimpleNamespace(**{k: g[k] for k in g.files})
+
+
+def _c1_sampled_gradients_close(ref, got_by_name, rtol, allow_few):
+    """Each hook gradient on the stored rows (``got_by_name[name]``: all in-frustum rows) and its L1 norm over all of them."""
+    for name, got in got_by_name.items():
+        exp = getattr(ref, "rows_hook_" + name)
+        sampled = got[ref.point_rows]
+        ok, (worst, nviol) = _close(sampled, exp, rtol=rtol, floor=1e-5)
+        # GPU / emulated CUDA: float32 atomics -- a few entries in a thousand may leave the per-entry tolerance, none by more
+        # than 1e-3 of the largest entry
+        assert ok or (allow_few and nviol <= 2e-3 * exp.size and np.abs(sampled - exp).max() <= 1e-3 * np.abs(exp).max()), \
+            (name, worst, nviol)
+        l1 = float(np.abs(got.astype(np.float64)).sum())
+        assert abs(l1 - float(getattr(ref, "l1_hook_" + name)[0])) <= rtol * l1, name
 
 
 def test_oracle_reproduces_the_reference_kernels_at_baseline_config_1():
@@ -176,26 +205,26 @@ def test_oracle_reproduces_the_reference_kernels_at_baseline_config_1():
     o, fwd, feats = oracle_forward(scene)
     assert np.array_equal(fwd.point_id_in_camera_list, ref.hook_point_id_in_camera_list) and fwd.point_id_in_camera_list.shape[0] == 9566
     assert np.array_equal(fwd.num_overlap_tiles, ref.hook_num_overlap_tiles)
-    assert np.array_equal(fwd.point_in_camera_sort_key, ref.stage_point_in_camera_sort_key)
-    assert np.array_equal(fwd.point_offset_with_sort_key, ref.stage_point_offset_with_sort_key)
+    assert np.array_equal(_digest(fwd.point_in_camera_sort_key), ref.sha256_stage_point_in_camera_sort_key)
+    assert np.array_equal(_digest(fwd.point_offset_with_sort_key), ref.sha256_stage_point_offset_with_sort_key)
     assert np.array_equal(fwd.tile_points_start, ref.stage_tile_points_start)
     assert np.array_equal(fwd.tile_points_end, ref.stage_tile_points_end)
     assert np.array_equal(fwd.pixel_valid_point_count, ref.count)
-    assert np.array_equal(fwd.pixel_offset_of_last_effective_point, ref.stage_pixel_offset_of_last_effective_point)
-    assert np.abs(fwd.image - ref.image).max() <= 5e-7 and (fwd.image == ref.image).mean() >= 0.99
-    assert np.abs(fwd.depth - ref.depth).max() <= 1e-4
-    assert np.abs(fwd.pixel_accumulated_alpha - ref.stage_pixel_accumulated_alpha).max() <= 2e-6
-    for got, exp in ((fwd.point_uv, ref.stage_point_uv), (fwd.point_uv_conic_and_rescale, ref.stage_point_uv_conic_and_rescale),
-                     (fwd.point_alpha_after_activation, ref.stage_point_alpha_after_activation),
-                     (fwd.point_color, ref.stage_point_color), (fwd.point_radii, ref.stage_point_radii)):
-        assert np.array_equal(got, exp)  # the per-point stage is bit-identical (see above)
+    assert np.array_equal(_digest(fwd.pixel_offset_of_last_effective_point), ref.sha256_stage_pixel_offset_of_last_effective_point)
+    pix = ref.pixel_index
+    image = fwd.image.reshape(-1, 3)[pix]
+    assert np.abs(image - ref.pixel_image).max() <= 5e-7 and (image == ref.pixel_image).mean() >= 0.99
+    assert np.abs(_tile_sums(fwd.image) - ref.tile_image_sum).max() <= 256 * 5e-7 + 1e-4  # + float32 rounding of the stored sums
+    assert np.abs(fwd.depth.reshape(-1, 1)[pix] - ref.pixel_depth).max() <= 1e-4
+    assert np.abs(fwd.pixel_accumulated_alpha.reshape(-1, 1)[pix] - ref.pixel_stage_pixel_accumulated_alpha).max() <= 2e-6
+    for key in C1_PER_POINT_STAGE:  # the per-point stage is bit-identical (see above)
+        assert np.array_equal(_digest(getattr(fwd, key)), getattr(ref, "sha256_stage_" + key)), key
     bwd = oracle_backward(o, fwd, scene, feats, _grad_image(sc).numpy(), 0)
     ids = ref.hook_point_id_in_camera_list.astype(np.int64)
-    for got, exp in ((bwd.grad_pointcloud[ids], ref.hook_grad_point_in_camera),
-                     (bwd.grad_pointcloud_features[ids], ref.hook_grad_pointfeatures_in_camera),
-                     (bwd.grad_viewspace, ref.hook_grad_viewspace), (bwd.magnitude_grad_viewspace, ref.hook_magnitude_grad_viewspace)):
-        ok, info = _close(got, exp, rtol=1e-4, floor=1e-5)
-        assert ok, info
+    _c1_sampled_gradients_close(ref, {"grad_point_in_camera": bwd.grad_pointcloud[ids],
+                                      "grad_pointfeatures_in_camera": bwd.grad_pointcloud_features[ids],
+                                      "grad_viewspace": bwd.grad_viewspace, "magnitude_grad_viewspace": bwd.magnitude_grad_viewspace},
+                                rtol=1e-4, allow_few=False)
     assert np.array_equal(bwd.num_affected_pixels, ref.hook_num_affected_pixels)
 
 
@@ -210,8 +239,10 @@ def test_cuda_operator_reproduces_the_reference_kernels_at_baseline_config_1(exa
     hook = {}
     op = make_op(hook=lambda h: hook.update(h=h), exact_exp=exact_exp)
     image, depth, count = run_forward(op, scene, band=0)
-    assert np.abs(n(image) - ref.image).max() <= 1e-4
-    assert np.abs(n(depth) - ref.depth).max() <= 1e-3
+    pix = ref.pixel_index
+    assert np.abs(n(image).reshape(-1, 3)[pix] - ref.pixel_image).max() <= 1e-4
+    assert np.abs(_tile_sums(n(image)) - ref.tile_image_sum).max() <= 256 * 1e-4
+    assert np.abs(n(depth).reshape(-1, 1)[pix] - ref.pixel_depth).max() <= 1e-3
     assert (n(count) != ref.count).sum() <= 3
     image.backward(_grad_image(sc).cuda())
     h = hook["h"]
@@ -219,12 +250,10 @@ def test_cuda_operator_reproduces_the_reference_kernels_at_baseline_config_1(exa
     assert np.array_equal(n(h.num_overlap_tiles), ref.hook_num_overlap_tiles)
     assert (n(h.num_affected_pixels) != ref.hook_num_affected_pixels).sum() <= 3
     ids = torch.from_numpy(ref.hook_point_id_in_camera_list.astype(np.int64)).cuda()
-    for got, exp in ((scene.point_cloud.grad[ids], ref.hook_grad_point_in_camera),
-                     (scene.point_cloud_features.grad[ids], ref.hook_grad_pointfeatures_in_camera),
-                     (h.grad_viewspace, ref.hook_grad_viewspace), (h.magnitude_grad_viewspace, ref.hook_magnitude_grad_viewspace)):
-        got = n(got)
-        ok, (worst, nviol) = _close(got, exp, rtol=1e-3, floor=1e-5)
-        assert ok or (nviol <= 2e-3 * exp.size and np.abs(got - exp).max() <= 1e-3 * np.abs(exp).max()), (worst, nviol)
+    _c1_sampled_gradients_close(ref, {"grad_point_in_camera": n(scene.point_cloud.grad[ids]),
+                                      "grad_pointfeatures_in_camera": n(scene.point_cloud_features.grad[ids]),
+                                      "grad_viewspace": n(h.grad_viewspace), "magnitude_grad_viewspace": n(h.magnitude_grad_viewspace)},
+                                rtol=1e-3, allow_few=True)
     rest = torch.ones(scene.point_cloud.shape[0], dtype=torch.bool, device="cuda")
     rest[ids] = False
     assert float(scene.point_cloud.grad[rest].abs().max()) == 0.0 and float(scene.point_cloud_features.grad[rest].abs().max()) == 0.0
@@ -235,14 +264,12 @@ def test_cuda_operator_reproduces_the_reference_kernels_at_baseline_config_1(exa
 # 976 x 544 = 2074 tiles with C2's splat density per tile.  Everything that must be bit-equal is stored as a SHA-256,
 # images and gradients as samples (6000 pixels, per-tile sums, 1500 in-frustum rows, global L1 norms).
 def _c2r():
-    import hashlib
     from reference_path_scenes import reduced_config_2
     path = os.path.join(HERE, "golden", "reference_path_c2_reduced.npz")
     if not os.path.exists(path):
         pytest.skip("reference_path_c2_reduced.npz has not been generated")
     g = np.load(path)
-    digest = lambda a: np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), dtype=np.uint8)  # noqa: E731
-    return reduced_config_2(), SimpleNamespace(**{k: g[k] for k in g.files}), digest
+    return reduced_config_2(), SimpleNamespace(**{k: g[k] for k in g.files}), _digest
 
 
 def test_oracle_reproduces_the_reference_kernels_at_reduced_config_2():
