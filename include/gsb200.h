@@ -87,7 +87,9 @@ typedef struct GsbWorkspaceLayout {
     int64_t keys_a, keys_b;    /* sort keys, key_bytes each, key_capacity_padded entries: a = as emitted (never written by
                                   the sort), b = sorted (whatever the number of radix passes that ran) */
     int64_t vals_a, vals_b;    /* int32 payload = in-camera offset, GPCR:930 */
-    int64_t keys_c, vals_c;    /* scratch of the radix passes (third buffer of the a -> [c -> b ->] ... -> b rotation) */
+    int64_t keys_c, vals_c;    /* scratch of the radix passes (third buffer of the a -> [c -> b ->] ... -> b rotation); after
+                                  the sort the forward blend (unless rgb_only) reuses keys_c for one uint8 per sorted key: the
+                                  mask of the 8x4-pixel patches of its tile that the splat can reach, read by the backward */
     int32_t key_bytes;         /* 4 or 8 */
     int32_t tile_bits, depth_bits, sort_passes;
     int64_t key_capacity_padded;

@@ -110,7 +110,7 @@ def main():
         "forward": {"visits": int(fw[7]), "pairs_with_alpha_above_cutoff_on_live_pixels": int(fw[8]),
                     "evaluated_pixel_splat_pairs": int(fw[7]) * 32, "scale_to_frame": round(float(T) / tiles.shape[0], 2)},
         "transposed": {"splat_visits": int(tb[3]), "chunks": int(tb[4]), "mean_chunk_fill": round(float(tb[3]) / max(int(tb[4]), 1), 2),
-                       "rows_flushed": int(tb[5]), "staging_batches": int(tb[6])},
+                       "rows_flushed": int(tb[5]), "windows": int(tb[6])},
         "estimated_warp_instructions_in_the_visit_loops": {"butterfly": int(est_bf), "transposed": int(est_tb),
                                                            "ratio": round(float(est_tb) / max(float(est_bf), 1.0), 3)},
         "note": "counts from the kernel sources under the CPU emulator; instruction weights from SASS; NOT a time measurement"}))

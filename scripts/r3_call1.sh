@@ -1,0 +1,35 @@
+#!/bin/bash
+# round 3, call 1 (1 GPU): loop A of the backward walking the reach masks the forward records, against the parent commit's
+# library (built from the parent's sources as libgsb200_parent.so), alternated three times; the 4-CTAs-per-SM variant build;
+# the GPU suite and smoke(); the outputs of both builds compared.
+set -u
+OUT=${1:?usage: bash $0 OUTPUT_DIR}  # logs and output dumps go here
+mkdir -p "$OUT"
+export PYTHONUNBUFFERED=1
+P=$PWD/taichi_3d_gaussian_splatting_b200/libgsb200_parent.so
+V=$PWD/taichi_3d_gaussian_splatting_b200/libgsb200_mb4.so
+BENCH="python bench.py --gpus 1 --steps 200 --warmup 20 --repeats 4 --no-cpu-baseline"
+DUMP="python bench.py --gpus 1 --steps 20 --warmup 5 --no-cpu-baseline"
+{
+nvidia-smi --query-gpu=name,power.limit,clocks.max.sm --format=csv
+echo "== build + smoke"; timeout 900 python -c "import __graft_entry__ as g; g.build(); g.smoke()" 2>&1 | tail -3
+for r in 1 2 3; do
+  echo "== round $r parent"
+  GSB200_LIB_PATH=$P timeout 300 $BENCH
+  GSB200_LIB_PATH=$P timeout 300 python scripts/bench_stages.py C3
+  echo "== round $r new"
+  timeout 300 $BENCH
+  timeout 300 python scripts/bench_stages.py C3
+done
+echo "== variant GSB_TB_MIN_BLOCKS=4"
+GSB200_LIB_PATH=$V timeout 300 $BENCH
+GSB200_LIB_PATH=$V timeout 300 python scripts/bench_stages.py C3
+echo "== output dumps"
+GSB200_LIB_PATH=$P timeout 300 $DUMP --dump-outputs "$OUT/dump_parent_a" | tail -1
+GSB200_LIB_PATH=$P timeout 300 $DUMP --dump-outputs "$OUT/dump_parent_b" | tail -1
+timeout 300 $DUMP --dump-outputs "$OUT/dump_new" | tail -1
+python scripts/compare_dumps.py "$OUT/dump_parent_a" "$OUT/dump_parent_b" "$OUT/dump_new"
+echo "== gpu tests"; timeout 1800 python -m pytest tests -q -m gpu -p no:cacheprovider 2>&1 | tail -8
+nvidia-smi --query-gpu=name,power.limit,clocks.max.sm --format=csv
+} 2>&1 | tee "$OUT/r3_call1.log"
+rm -rf "$OUT/dump_parent_a" "$OUT/dump_parent_b" "$OUT/dump_new"

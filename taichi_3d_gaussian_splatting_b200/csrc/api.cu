@@ -130,6 +130,7 @@ int resolve_workspace(void *base, int64_t bytes, int64_t N, int32_t n_obj, int64
     ws->vals_b = reinterpret_cast<int *>(b + L.vals_b);
     ws->keys_c = b + L.keys_c;
     ws->vals_c = reinterpret_cast<int *>(b + L.vals_c);
+    ws->patch_masks = reinterpret_cast<unsigned char *>(b + L.keys_c);  // key_capacity_padded * key_bytes >= one byte per key
     return GSB_OK;
 }
 

@@ -273,6 +273,7 @@ static BlendBwdParams make_blend_bwd_params(const GsbBackwardArgs &a, const Work
     p.grad_image = a.grad_rasterized_image;
     p.acc_alpha = a.pixel_accumulated_alpha;
     p.last_effective = a.pixel_offset_of_last_effective_point;
+    p.patch_masks = ws.patch_masks;
     p.accum = a.accum;
     p.mag_image = a.magnitude_grad_viewspace_on_image;
     p.work_counters = nullptr;
@@ -291,6 +292,7 @@ int launch_blend_backward(const GsbBackwardArgs &a, const Workspace &ws, cudaStr
     p.grad_image = a.grad_rasterized_image;
     p.acc_alpha = a.pixel_accumulated_alpha;
     p.last_effective = a.pixel_offset_of_last_effective_point;
+    p.patch_masks = ws.patch_masks;
     p.accum = a.accum;
     p.mag_image = a.magnitude_grad_viewspace_on_image;
     p.work_counters = nullptr;

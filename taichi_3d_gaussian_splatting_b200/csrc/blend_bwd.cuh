@@ -14,6 +14,7 @@ struct BlendBwdParams {
     const float *grad_image;
     const float *acc_alpha;
     const int *last_effective;
+    const unsigned char *patch_masks = nullptr;  // the forward's reach mask per sorted key (blend_bwd_transposed.cu only)
     float *accum;      // rows of 12 floats
     float *mag_image;  // (H,W,2)
     unsigned long long *work_counters;  // COUNT instantiation only: [0] (warp, splat) visits, [1] contributing (pixel, splat) pairs

@@ -27,6 +27,7 @@ struct BlendFwdParams {
     float *acc_alpha;
     int *last_effective;
     int *valid_count;
+    unsigned char *patch_masks = nullptr;  // !RGB_ONLY: the reach mask of every staged key, by sorted index (read by the backward)
     unsigned long long *work_counters;  // COUNT instantiation only: [0] (warp, splat) visits, [1] (pixel, splat)
                                         //   evaluations with alpha >= 1/255 on a live pixel (SURVEY 8(d) "E"); what-if
                                         //   counters at staging time (before any saturation exit): [2] (8x4 patch, splat)
@@ -35,6 +36,17 @@ struct BlendFwdParams {
 };
 
 __device__ __forceinline__ float ex2_approx(float x) { return ex2_mufu(x); }
+
+#ifdef GSB_HOST_EMU
+// tests/simt: the entry points that run the forward blend on its own pass no mask array
+inline void store_patch_mask(unsigned char *masks, int idx, unsigned int mask) {
+    if (masks) masks[idx] = (unsigned char)mask;
+}
+#else
+__device__ __forceinline__ void store_patch_mask(unsigned char *masks, int idx, unsigned int mask) {
+    masks[idx] = (unsigned char)mask;
+}
+#endif
 
 // cnt += 1 and last = idx for a blended pair (wgt > 0): one FSETP and two predicated moves instead of the four instructions
 // the compiler makes of the two selects
@@ -118,6 +130,9 @@ blend_forward_kernel(const BlendFwdParams p) {
             }
             s_r2[tid] = __ldg(rec + 2);
             mask = splat_patch_mask(r0.x, r0.y, r0.z, r0.w, r1.x, r1.y * r1.z, tile_x0, tile_y0);
+            // the backward walks the keys below each patch's deepest effective splat; all of them are staged here (the
+            // early exit below comes after the staging of its batch)
+            if (!RGB_ONLY) store_patch_mask(p.patch_masks, idx, mask);
             if (COUNT) {  // patch w sits at column (w & 1), row (w >> 1)
                 n_p84 += __popc(mask);
                 n_p88 += __popc((mask | (mask >> 2)) & 0x33u);   // rows 0|1 and 2|3 merged
@@ -266,6 +281,7 @@ int launch_blend_forward(const GsbForwardArgs &a, const Workspace &ws, cudaStrea
     p.acc_alpha = a.pixel_accumulated_alpha;
     p.last_effective = a.pixel_offset_of_last_effective_point;
     p.valid_count = a.pixel_valid_point_count;
+    p.patch_masks = ws.patch_masks;
     p.work_counters = nullptr;
     const int tiles = p.tiles_x * (a.camera_height / GSB_TILE_HEIGHT);
     if (tiles <= 0) return GSB_OK;
@@ -299,6 +315,7 @@ int launch_blend_forward_count(const GsbForwardArgs &a, const Workspace &ws, uns
     p.acc_alpha = a.pixel_accumulated_alpha;
     p.last_effective = a.pixel_offset_of_last_effective_point;
     p.valid_count = a.pixel_valid_point_count;
+    p.patch_masks = ws.patch_masks;
     p.work_counters = counters_dev;
     const int tiles = p.tiles_x * (a.camera_height / GSB_TILE_HEIGHT);
     if (tiles <= 0) return GSB_OK;

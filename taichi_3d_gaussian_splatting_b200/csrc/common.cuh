@@ -54,6 +54,8 @@ struct Workspace {
     float *point_in_camera; // 3 floats per in-camera point
     void *keys_a, *keys_b, *keys_c;  // emitted keys (a), sorted keys (b), scratch of the radix passes (c)
     int *vals_a, *vals_b, *vals_c;
+    unsigned char *patch_masks;  // one byte per sorted key: the 8-patch reach mask the forward blend computed for it
+                                 //   (bit w = patch of warp w); lives in keys_c, which is dead once the sort has finished
     GsbWorkspaceLayout layout;
 };
 
@@ -242,6 +244,12 @@ __device__ __forceinline__ void bulk_copy_g2s(void *dst_smem, const void *src_gm
 // every lane of the warp calls the wait (warp-uniform condition at both call sites): under the emulator it is a warp
 // rendezvous, so the lane that issued the (immediate) copy has done so before any lane reads the destination
 __device__ __forceinline__ void mbar_wait(unsigned long long *, unsigned int) { simt_emu::warp_exchange(0u); }
+// cp.async (16-byte global -> shared copies, per-thread groups): the copy lands at once; the wait is called by every lane
+// of the warp and is a warp rendezvous, as above
+__device__ __forceinline__ void cp_async16(void *dst_smem, const void *src_gmem) { memcpy(dst_smem, src_gmem, 16); }
+__device__ __forceinline__ void cp_async_commit() {}
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { simt_emu::warp_exchange(0u); }
 #else
 // ---- mbarrier / bulk-copy helpers (TMA 1-D bulk copy, global -> shared)
 __device__ __forceinline__ unsigned int smem_addr(const void *p) {
@@ -277,6 +285,17 @@ __device__ __forceinline__ void mbar_wait(unsigned long long *bar, unsigned int 
         "r"(parity)
         : "memory");
 }
+// ---- cp.async: 16-byte global -> shared copy through L1 (.ca: the CTA's other warps read the same records), in per-thread
+// groups.  After cp_async_wait<N>() the thread's own copies of all but the N most recent groups have landed; a __syncwarp()
+// then makes them visible to the rest of the warp.
+__device__ __forceinline__ void cp_async16(void *dst_smem, const void *src_gmem) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_addr(dst_smem)), "l"(src_gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() {
+    asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
+}
 #endif
 
 #endif
@@ -294,7 +313,7 @@ enum EmuCounter {
     EC_TB_SPLATS = 3,       // transposed kernel: (warp, splat) list entries
     EC_TB_CHUNKS = 4,       //   chunks processed
     EC_TB_ROWS = 5,         //   accumulator rows flushed (splats with a contributing pixel)
-    EC_BATCHES = 6,         // staging batches (per CTA)
+    EC_TB_WINDOWS = 6,      //   32-key windows of the sorted list walked (per warp)
     EC_FW_VISITS = 7,       // forward blend: (warp, splat) visits
     EC_FW_PAIRS = 8,        //   (pixel, splat) pairs with alpha >= 1/255 on a live pixel (blended or saturating)
 };
