@@ -60,6 +60,8 @@ enum {
                                             the reference's need_extra_info = False, GPCR:521, 690-704.  accum[:, 9:11] and
                                             magnitude_grad_viewspace_on_image are then left untouched (the pointer must still be valid) */
 
+#define GSB_POSE_MAX_OBJECTS 16          /* gsb200_backward_with_pose: most objects (pose rows) one call can differentiate */
+
 #define GSB_FLAG_COMPACT_GRADS 64u        /* backward only (view-parallel training, parallel.py): the per-point kernel writes
                                             grad_sum_compact (N,12) and grad_color_compact (N,3) instead of the dense
                                             gradients; gsb200_expand_view_gradients rebuilds them after the exchange */
@@ -175,6 +177,21 @@ typedef struct GsbBackwardArgs {
     float *ctl_accumulated_position_gradients_norm;
 } GsbBackwardArgs;
 
+/* Gradients of the per-object camera poses (the q_pointcloud_camera / t_pointcloud_camera slots of GPCR:1027, 1157-1163,
+ * which the reference declares and leaves empty), for gsb200_backward_with_pose.  They are the gradients of the same surrogate
+ * the xyz and feature gradients differentiate (J inside Sigma', the SH view direction and `rescale` held fixed, the 0.99 clamp
+ * straight through): the pose reaches the image through the point means p_cam = W x + t_c and through the rotation of the
+ * covariance, U = J W, with W = the rotation polynomial of conj(q) as given and t_c = -rotate(conj(q) / |conj(q)|, t), exactly
+ * as the forward builds them.  Per view: a view-parallel (GSB_FLAG_COMPACT_GRADS) call returns this view's pose gradients. */
+typedef struct GsbPoseGradArgs {
+    const float *q_pointcloud_camera;  /* (num_objects,4) the forward's */
+    const float *t_pointcloud_camera;  /* (num_objects,3) the forward's */
+    float *grad_q_pointcloud_camera;   /* (num_objects,4) out, fully written (zeros for an object with no point in the frustum) */
+    float *grad_t_pointcloud_camera;   /* (num_objects,3) out, fully written */
+    void *temp;                        /* >= gsb200_pose_grad_temp_bytes(num_objects) bytes, 16-byte aligned; no initialisation */
+    int64_t temp_bytes;
+} GsbPoseGradArgs;
+
 /* View-parallel training (SURVEY 8(e); the reference is single-GPU): after the ranks have exchanged their COMPACT rows --
  * all-reduce(sum) of grad_sum_compact, all-gather of [grad_color_compact | t_pointcloud_camera] -- rebuild the dense
  * gradients of the whole batch of views: (N,3) and (N,56) exactly as the sum over views of what gsb200_backward writes
@@ -206,7 +223,8 @@ const char *gsb200_last_error(void);
 /* sizeof(GsbWorkspaceLayout), sizeof(GsbForwardArgs), sizeof(GsbBackwardArgs) as compiled: lets a
  * foreign-language binding verify its struct mirrors. */
 void gsb200_abi_sizes(int64_t *out3);
-/* ... and of the first n of {GsbWorkspaceLayout, GsbForwardArgs, GsbBackwardArgs, GsbExpandArgs, GsbTrainStepArgs} */
+/* ... and of the first n of {GsbWorkspaceLayout, GsbForwardArgs, GsbBackwardArgs, GsbExpandArgs, GsbTrainStepArgs,
+ * GsbPoseGradArgs} */
 void gsb200_abi_sizes_ext(int64_t *out, int32_t n);
 
 /* Workspace sizing.  far_plane*depth_to_sort_key_scale fixes the depth-key width; (H/16)*(W/16)
@@ -234,6 +252,14 @@ int gsb200_forward(const GsbForwardArgs *args);
 int gsb200_backward(const GsbBackwardArgs *args);
 
 int gsb200_expand_view_gradients(const GsbExpandArgs *args);
+
+/* gsb200_backward plus the gradients of the object poses (GsbPoseGradArgs): every output of gsb200_backward is computed as it
+ * computes it, bit for bit, and the pose gradients are summed in a fixed order (deterministic).  args->num_objects poses;
+ * GSB_EUNSUPPORTED above GSB_POSE_MAX_OBJECTS, GSB_EINVAL for a null pointer or a short temp -- both checked before anything
+ * is enqueued.  The pose part adds a second instantiation of the per-point kernel and one small finalisation kernel.
+ * (Present since version 102; detect it by the symbol.) */
+int64_t gsb200_pose_grad_temp_bytes(int32_t num_objects);
+int gsb200_backward_with_pose(const GsbBackwardArgs *args, const GsbPoseGradArgs *pose);
 
 /* The two collectives of the compact exchange as ONE hand-written kernel over NVSwitch multicast memory (NVLS; csrc/exchange.cu):
  * a two-shot all-reduce of grad_sum (multimem.ld_reduce of this rank's 1/R of the rows, multimem.st of the sums to all ranks)

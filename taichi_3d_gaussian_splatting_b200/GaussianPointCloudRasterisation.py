@@ -12,7 +12,10 @@ for device memory, streams and autograd plumbing.  There is no CPU fallback.
 Contract details kept from the reference (SURVEY.md §8(b), §9):
 * in-frustum rows of ``point_cloud_features[:, 0:4]`` are normalised IN PLACE each forward
   (GPCR:264-266);
-* backward does nothing (all ``None``) unless xyz or features require grad (GPCR:1028);
+* backward does nothing (all ``None``) unless xyz, features or a pose requires grad (GPCR:1028);
+* the pose gradients, which the reference declares and leaves ``None`` (GPCR:1027, 1157-1163), are filled
+  (``gsb200_backward_with_pose``) when ``q_pointcloud_camera`` or ``t_pointcloud_camera`` requires grad -- the gradient of
+  the same surrogate the xyz gradient follows (DESIGN.md §9); a pose-only backward does not call the hook;
 * the hook runs synchronously inside backward, after gradient scaling (GPCR:1127-1142);
 * ``grad_*_factor`` are un-annotated class constants, i.e. not dataclass fields (GPCR:782-786);
 * ``camera_width`` / ``camera_height`` must be multiples of 16 (GPCR:1193-1194).
@@ -277,24 +280,35 @@ class GaussianPointCloudRasterisation(torch.nn.Module):
                 image, depth, acc_alpha, last_effective, valid_count = outs
                 ctx.save_for_backward(pointcloud, pointcloud_features, point_object_id,
                                       t_pointcloud_camera, saved["camera_intrinsics"], acc_alpha,
-                                      last_effective, frame.ws)
+                                      last_effective, frame.ws, saved["q_pointcloud_camera"])
                 ctx.frame = frame
                 ctx.num_objects = q_pointcloud_camera.shape[0]
+                ctx.q_shape, ctx.t_shape = q_pointcloud_camera.shape, t_pointcloud_camera.shape
                 ctx.color_max_sh_band = color_max_sh_band
                 ctx.mark_non_differentiable(depth, valid_count)
                 return image, depth, valid_count
 
             @staticmethod
             def backward(ctx, grad_rasterized_image, grad_rasterized_depth, grad_pixel_valid_point_count):
-                grad_pointcloud = grad_pointcloud_features = None
-                if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:  # GPCR:1028
+                grad_pointcloud = grad_pointcloud_features = grad_q = grad_t = None
+                scene = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]  # GPCR:1028
+                pose = ctx.needs_input_grad[4] or ctx.needs_input_grad[5]
+                if scene or pose:
                     if outer.config.rgb_only:
                         # the reference leaves accumulated alpha / last-effective offsets uninitialised in
                         # this mode (GPCR:478-484), so its backward is undefined; refuse instead
                         raise RuntimeError("rgb_only=True is an inference-only mode: backward needs the "
                                            "auxiliary per-pixel outputs")
-                    grad_pointcloud, grad_pointcloud_features = outer._run_backward(ctx, grad_rasterized_image)
-                return grad_pointcloud, grad_pointcloud_features, None, None, None, None, None, None
+                    if pose:
+                        grad_pointcloud, grad_pointcloud_features, grad_q, grad_t = outer._run_backward(
+                            ctx, grad_rasterized_image, pose=True, scene=scene)
+                        if not scene:  # tracking against a frozen scene: no scene gradients, no hook
+                            grad_pointcloud = grad_pointcloud_features = None
+                        grad_q = grad_q.view(ctx.q_shape) if ctx.needs_input_grad[4] else None
+                        grad_t = grad_t.view(ctx.t_shape) if ctx.needs_input_grad[5] else None
+                    else:
+                        grad_pointcloud, grad_pointcloud_features = outer._run_backward(ctx, grad_rasterized_image)
+                return grad_pointcloud, grad_pointcloud_features, None, None, grad_q, grad_t, None, None
 
         self._module_function = _module_function
 
@@ -391,14 +405,17 @@ class GaussianPointCloudRasterisation(torch.nn.Module):
             finally:  # also when the library call raises: the pooled pair goes back
                 _PinnedCounters.release(device, readback)
         self.last_frame = frame
-        return (image, depth, acc_alpha, last_effective, valid_count), frame, {"camera_intrinsics": K}
+        return (image, depth, acc_alpha, last_effective, valid_count), frame, {"camera_intrinsics": K,
+                                                                               "q_pointcloud_camera": q_pc}
 
     # ------------------------------------------------------------------ backward plumbing
-    def _run_backward(self, ctx, grad_rasterized_image):
+    def _run_backward(self, ctx, grad_rasterized_image, pose: bool = False, scene: bool = True):
+        """Dense gradients (and the hook).  ``pose``: also the gradients of q / t_pointcloud_camera (gsb200_backward_with_pose),
+        returned as two more tensors; ``scene = False`` (pose only): the hook is not called and no gradient is exchanged."""
         cfg = self.config
         lib = _lib.load()
         (pointcloud, pointcloud_features, point_object_id, t_pointcloud_camera, K, acc_alpha,
-         last_effective, ws) = ctx.saved_tensors
+         last_effective, ws, q_pointcloud_camera) = ctx.saved_tensors
         frame: Frame = ctx.frame
         device = pointcloud.device
         N = pointcloud.shape[0]
@@ -425,7 +442,7 @@ class GaussianPointCloudRasterisation(torch.nn.Module):
             t_pc = t_pointcloud_camera.contiguous()
             backward_flags = self.backward_flags(frame.flags)
             exchange = self.gradient_exchange
-            compact = exchange is not None and exchange.world > 1
+            compact = exchange is not None and exchange.world > 1 and scene
             grad_sum = blocks = None
             if compact:
                 n_obj = ctx.num_objects
@@ -447,7 +464,24 @@ class GaussianPointCloudRasterisation(torch.nn.Module):
                 grad_pointcloud_features=_ptr(grad_pointcloud_features),
                 magnitude_grad_viewspace_on_image=_ptr(magnitude_on_image), stream=stream.cuda_stream,
                 grad_sum_compact=_ptr(grad_sum), grad_color_compact=_ptr(blocks[exchange.rank]) if compact else None)
-            _lib.check(lib.gsb200_backward(ctypes.byref(args)), "gsb200_backward")
+            if pose:
+                n_obj = ctx.num_objects
+                if not hasattr(lib, "gsb200_backward_with_pose"):
+                    raise RuntimeError(f"{_lib.LIB_PATH} has no gsb200_backward_with_pose: rebuild it for pose gradients")
+                if n_obj > _lib.GSB_POSE_MAX_OBJECTS:
+                    raise RuntimeError(f"pose gradients are available for at most {_lib.GSB_POSE_MAX_OBJECTS} objects, "
+                                       f"got {n_obj}")
+                grad_pose = torch.empty((7 * n_obj,), dtype=torch.float32, device=device)
+                grad_q, grad_t = grad_pose[:4 * n_obj].view(n_obj, 4), grad_pose[4 * n_obj:].view(n_obj, 3)
+                temp = torch.empty((lib.gsb200_pose_grad_temp_bytes(n_obj),), dtype=torch.uint8, device=device)
+                pargs = _lib.GsbPoseGradArgs(
+                    q_pointcloud_camera=_ptr(q_pointcloud_camera), t_pointcloud_camera=_ptr(t_pc),
+                    grad_q_pointcloud_camera=_ptr(grad_q), grad_t_pointcloud_camera=_ptr(grad_t), temp=_ptr(temp),
+                    temp_bytes=temp.numel())
+                _lib.check(lib.gsb200_backward_with_pose(ctypes.byref(args), ctypes.byref(pargs)),
+                           "gsb200_backward_with_pose")
+            else:
+                _lib.check(lib.gsb200_backward(ctypes.byref(args)), "gsb200_backward")
             own_view_grad_xyz = None
             if compact:
                 exchange.rows_written(grad_sum, blocks)
@@ -469,7 +503,7 @@ class GaussianPointCloudRasterisation(torch.nn.Module):
 
                 exchange.run_and_expand(grad_sum, blocks, expand)
 
-            hook = self.backward_valid_point_hook
+            hook = self.backward_valid_point_hook if scene else None
             if hook is not None:  # GPCR:1127-1142
                 ids = frame.point_id_in_camera_list
                 ids64 = ids.long()
@@ -486,6 +520,8 @@ class GaussianPointCloudRasterisation(torch.nn.Module):
                     point_uv_in_camera=frame.point_uv.contiguous(),
                     point_depth=frame.point_in_camera[:, 2],
                 ))
+        if pose:
+            return grad_pointcloud, grad_pointcloud_features, grad_q, grad_t
         return grad_pointcloud, grad_pointcloud_features
 
     def backward_flags(self, frame_flags: int) -> int:

@@ -93,6 +93,15 @@ class GsbExpandArgs(ctypes.Structure):
     ]
 
 
+class GsbPoseGradArgs(ctypes.Structure):
+    _fields_ = [
+        ("q_pointcloud_camera", c_vp), ("t_pointcloud_camera", c_vp), ("grad_q_pointcloud_camera", c_vp),
+        ("grad_t_pointcloud_camera", c_vp), ("temp", c_vp), ("temp_bytes", c_i64),
+    ]
+
+
+GSB_POSE_MAX_OBJECTS = 16
+
 EXPORTS = (
     "gsb200_version", "gsb200_last_error", "gsb200_workspace_layout", "gsb200_forward",
     "gsb200_backward", "gsb200_stage_preprocess", "gsb200_stage_sort", "gsb200_stage_tile_ranges",
@@ -100,7 +109,8 @@ EXPORTS = (
     "gsb200_forward_timed", "gsb200_backward_timed", "gsb200_abi_sizes", "gsb200_l1_loss_temp_bytes", "gsb200_l1_loss",
     "gsb200_image_loss_temp_bytes", "gsb200_image_loss", "gsb200_adam_step", "gsb200_controller_update",
     "gsb200_forward_blend_work", "gsb200_backward_blend_work", "gsb200_device_selftest", "gsb200_expand_view_gradients",
-    "gsb200_train_step", "gsb200_abi_sizes_ext", "gsb200_exchange_multimem",
+    "gsb200_train_step", "gsb200_abi_sizes_ext", "gsb200_exchange_multimem", "gsb200_pose_grad_temp_bytes",
+    "gsb200_backward_with_pose",
 )
 
 _lib = None
@@ -126,6 +136,12 @@ def load() -> ctypes.CDLL:
         getattr(lib, name).restype = ctypes.c_int
     lib.gsb200_backward.argtypes = [ctypes.POINTER(GsbBackwardArgs)]
     lib.gsb200_backward.restype = ctypes.c_int
+    has_pose = hasattr(lib, "gsb200_backward_with_pose")  # the pose gradients are detected by their symbol
+    if has_pose:
+        lib.gsb200_backward_with_pose.argtypes = [ctypes.POINTER(GsbBackwardArgs), ctypes.POINTER(GsbPoseGradArgs)]
+        lib.gsb200_backward_with_pose.restype = ctypes.c_int
+        lib.gsb200_pose_grad_temp_bytes.argtypes = [c_i32]
+        lib.gsb200_pose_grad_temp_bytes.restype = c_i64
     lib.gsb200_sort_temp_bytes.argtypes = [c_i64, c_i32]
     lib.gsb200_sort_temp_bytes.restype = c_i64
     lib.gsb200_sort_pairs.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_i32, c_i32, c_vp, c_i64, c_vp]
@@ -163,11 +179,12 @@ def load() -> ctypes.CDLL:
     if tuple(sizes) != mine:
         raise RuntimeError(f"libgsb200.so ABI mismatch: C struct sizes {tuple(sizes)} != ctypes mirrors {mine}; "
                            "rebuild with `python -m taichi_3d_gaussian_splatting_b200.build --force`")
-    sizes5 = (c_i64 * 5)()
-    lib.gsb200_abi_sizes_ext(sizes5, 5)
-    mine5 = mine + (ctypes.sizeof(GsbExpandArgs), ctypes.sizeof(GsbTrainStepArgs))
-    if tuple(sizes5) != mine5:
-        raise RuntimeError(f"libgsb200.so ABI mismatch: C struct sizes {tuple(sizes5)} != ctypes mirrors {mine5}")
+    n_ext = 6 if has_pose else 5
+    sizes_ext = (c_i64 * n_ext)()
+    lib.gsb200_abi_sizes_ext(sizes_ext, n_ext)
+    mine_ext = (mine + (ctypes.sizeof(GsbExpandArgs), ctypes.sizeof(GsbTrainStepArgs), ctypes.sizeof(GsbPoseGradArgs)))[:n_ext]
+    if tuple(sizes_ext) != mine_ext:
+        raise RuntimeError(f"libgsb200.so ABI mismatch: C struct sizes {tuple(sizes_ext)} != ctypes mirrors {mine_ext}")
     _lib = lib
     return lib
 

@@ -193,9 +193,9 @@ void gsb200_abi_sizes(int64_t *out3) {
 }
 
 void gsb200_abi_sizes_ext(int64_t *out, int32_t n) {
-    const int64_t all[5] = {(int64_t)sizeof(GsbWorkspaceLayout), (int64_t)sizeof(GsbForwardArgs), (int64_t)sizeof(GsbBackwardArgs),
-                            (int64_t)sizeof(GsbExpandArgs), (int64_t)sizeof(GsbTrainStepArgs)};
-    for (int i = 0; i < n && i < 5; ++i) out[i] = all[i];
+    const int64_t all[6] = {(int64_t)sizeof(GsbWorkspaceLayout), (int64_t)sizeof(GsbForwardArgs), (int64_t)sizeof(GsbBackwardArgs),
+                            (int64_t)sizeof(GsbExpandArgs), (int64_t)sizeof(GsbTrainStepArgs), (int64_t)sizeof(GsbPoseGradArgs)};
+    for (int i = 0; i < n && i < 6; ++i) out[i] = all[i];
 }
 
 int gsb200_workspace_layout(int64_t num_points, int32_t num_objects, int64_t key_capacity,
@@ -253,7 +253,7 @@ int gsb200_forward(const GsbForwardArgs *a) {
     return launch_blend_forward(*a, ws, st);
 }
 
-static int backward_impl(const GsbBackwardArgs *a, bool skip_on_overflow) {
+static int backward_impl(const GsbBackwardArgs *a, bool skip_on_overflow, const GsbPoseGradArgs *pose = nullptr) {
     if (!a) {
         set_error("backward: args is null");
         return GSB_EINVAL;
@@ -301,10 +301,36 @@ static int backward_impl(const GsbBackwardArgs *a, bool skip_on_overflow) {
     if (a->accum_rows > 0)
         GSB_CUDA_CHECK(cudaMemsetAsync(a->accum, 0, (size_t)a->accum_rows * GSB_ACCUM_FLOATS * 4, st));
     if ((rc = launch_blend_backward(*a, ws, st)) != GSB_OK) return rc;
-    return launch_backward_points(*a, ws, st, skip_on_overflow ? ws.counters + CNT_OVERFLOW : nullptr);
+    return launch_backward_points(*a, ws, st, skip_on_overflow ? ws.counters + CNT_OVERFLOW : nullptr, pose);
 }
 
 int gsb200_backward(const GsbBackwardArgs *a) { return backward_impl(a, false); }
+
+int64_t gsb200_pose_grad_temp_bytes(int32_t num_objects) {
+    return num_objects > 0 ? (int64_t)POSE_MAX_BLOCKS * num_objects * 12 * (int64_t)sizeof(float) : 0;
+}
+
+int gsb200_backward_with_pose(const GsbBackwardArgs *a, const GsbPoseGradArgs *pose) {
+    if (!a || !pose) {
+        set_error("backward_with_pose: args or pose is null");
+        return GSB_EINVAL;
+    }
+    if (a->num_objects > GSB_POSE_MAX_OBJECTS) {
+        set_error("backward_with_pose: %d objects, at most %d poses can be differentiated", a->num_objects, GSB_POSE_MAX_OBJECTS);
+        return GSB_EUNSUPPORTED;
+    }
+    if (a->num_objects < 1 || !pose->q_pointcloud_camera || !pose->t_pointcloud_camera || !pose->grad_q_pointcloud_camera ||
+        !pose->grad_t_pointcloud_camera || !pose->temp) {
+        set_error("backward_with_pose: null pointer argument or no object");
+        return GSB_EINVAL;
+    }
+    if (pose->temp_bytes < gsb200_pose_grad_temp_bytes(a->num_objects) || reinterpret_cast<uintptr_t>(pose->temp) % 16 != 0) {
+        set_error("backward_with_pose: temp must hold %lld bytes, 16-byte aligned (have %lld)",
+                  (long long)gsb200_pose_grad_temp_bytes(a->num_objects), (long long)pose->temp_bytes);
+        return GSB_EINVAL;
+    }
+    return backward_impl(a, false, pose);
+}
 
 int gsb200_image_loss(const float *rasterized_image, const float *ground_truth_image, int32_t camera_height,
                       int32_t camera_width, float lambda_value, float upstream_grad, float *loss_out3,

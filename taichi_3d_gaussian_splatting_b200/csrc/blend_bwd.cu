@@ -365,7 +365,52 @@ struct PointsBwdParams {
                                 //   controller accumulators alone (fused train step: the whole step becomes a no-op)
     float *grad_sum_compact;    // COMPACT: (N,12) xyz(3) q(4) s(3) logit(1) pad -- the columns that simply add up over views
     float *grad_color_compact;  // COMPACT: (N,3) d L / d (SH colour argument), per VIEW (its SH basis depends on the camera centre)
+    // POSE: per-CTA sums of the 12 pose values of every object -> pose_partials[block][obj][12] (pose_grad_finalize_kernel)
+    int pose_num_objects;       // <= GSB_POSE_MAX_OBJECTS
+    float *pose_partials;
 };
+
+// Sum 12 per-lane values over the warp with 13 shuffles (the transposing butterfly of warp_transpose_reduce11 with an even
+// split at every stage: 12 -> 6 -> 3 -> 2 -> 1).  On return v[0] of lane l holds the warp total of value reduce12_slot(l);
+// the lanes for which reduce12_writer(l) is true cover 0..11 exactly once.  Fixed shuffle pattern: deterministic.
+__device__ __forceinline__ void warp_transpose_reduce12(float (&v)[12], int lane) {
+    {
+        const bool hi = lane & 16;  // keeps values 6..11, partner keeps 0..5
+#pragma unroll
+        for (int i = 0; i < 6; ++i) {
+            const float send = hi ? v[i] : v[i + 6];
+            const float keep = hi ? v[i + 6] : v[i];
+            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
+        }
+    }
+    {
+        const bool hi = lane & 8;  // slots 3..5 vs 0..2
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            const float send = hi ? v[i] : v[i + 3];
+            const float keep = hi ? v[i + 3] : v[i];
+            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, 8);
+        }
+    }
+    {
+        const bool hi = lane & 4;  // slot 2 vs slot 0; slot 1 on both sides
+        const float send = hi ? v[0] : v[2];
+        const float keep = hi ? v[2] : v[0];
+        v[0] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
+        v[1] += __shfl_xor_sync(0xffffffffu, v[1], 4);
+    }
+    {
+        const bool hi = lane & 2;  // slot 1 vs slot 0
+        const float send = hi ? v[0] : v[1];
+        const float keep = hi ? v[1] : v[0];
+        v[0] = keep + __shfl_xor_sync(0xffffffffu, send, 2);
+    }
+    v[0] += __shfl_xor_sync(0xffffffffu, v[0], 1);
+}
+__device__ __forceinline__ int reduce12_slot(int lane) {
+    return ((lane & 16) ? 6 : 0) + ((lane & 8) ? 3 : 0) + ((lane & 2) ? 1 : ((lane & 4) ? 2 : 0));
+}
+__device__ __forceinline__ bool reduce12_writer(int lane) { return !(lane & 1) && !((lane & 2) && (lane & 4)); }
 
 #ifndef GSB_POINTS_THREADS
 #define GSB_POINTS_THREADS 128
@@ -377,8 +422,14 @@ constexpr int PT_ROW_COMPACT = 20;  // COMPACT: 16 staged floats per row, same b
 // applied -- and the 3 colour-argument gradients that must stay per view: the 48 SH gradients of a view are their outer product
 // with the view's SH basis, which gsb200_expand_view_gradients rebuilds AFTER the exchange (14 instead of 59 floats per row
 // cross NVLink, and this kernel writes 60 instead of 236 bytes per row).
-template <bool COMPACT>
-__global__ void __launch_bounds__(GSB_POINTS_THREADS, 6)  // 6 x 33 KB of staging per SM
+// POSE = true (gsb200_backward_with_pose): every in-frustum row also forms the 12 values through which the pose of its object
+// reaches the image under the same surrogate as the xyz gradient (DESIGN.md section 9): dL/dt_c (3) and dL/dW (9), with
+// p_cam = W x + t_c.  They are summed per object in a fixed order -- lanes grouped by object (__match_any_sync) and folded with
+// a fixed shuffle butterfly, groups added into per-warp shared slots, the warps added in warp order at the end of the CTA --
+// and written as pose_partials[block][obj][12]; pose_grad_finalize_kernel adds the blocks and applies the chain rule to (q, t).
+// Every other output is computed by the same code as with POSE = false.
+template <bool COMPACT, bool POSE = false>
+__global__ void __launch_bounds__(GSB_POINTS_THREADS, 6)  // 6 x 33 KB of staging per SM (+3 KB of pose slots with POSE)
 backward_points_kernel(const PointsBwdParams p) {
     // One thread per scene row: rows outside the frustum get their zeros here (no separate memset of the
     // dense (N,3)/(N,56) gradients), rows inside get the chain rule.  A warp owns 32 consecutive rows, i.e. one
@@ -391,10 +442,17 @@ backward_points_kernel(const PointsBwdParams p) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     float *const my_feat = &s_feat[warp][lane * ROW];
     float *const my_xyz = &s_xyz[warp][lane * 3];
+    __shared__ float s_pose[POSE ? GSB_POINTS_THREADS / 32 : 1][POSE ? GSB_POSE_MAX_OBJECTS : 1][12];
+    if (POSE) {  // each warp clears and later fills only its own slots
+        for (int k = lane; k < p.pose_num_objects * 12; k += 32) s_pose[warp][k / 12][k % 12] = 0.0f;
+        __syncwarp();
+    }
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long base = (long long)blockIdx.x * blockDim.x + warp * 32; base < p.N; base += stride) {
       const long long id = base + lane;
       const int o = id < p.N ? p.point_offset[id] : -1;
+      int pose_obj = -1;  // POSE: object of this lane's row if it is in the frustum
+      float pv[12];       // POSE: dL/dt_c (3) | dL/dW row-major (9) of this row
       if (o < 0) {
           if (!COMPACT) { my_xyz[0] = 0.0f; my_xyz[1] = 0.0f; my_xyz[2] = 0.0f; }
 #pragma unroll
@@ -499,6 +557,41 @@ backward_points_kernel(const PointsBwdParams p) {
             p.ctl_pos_grad[3 * id + 2] += gx[2];
             p.ctl_pos_grad_norm[id] += sqrtf(gx[0] * gx[0] + gx[1] * gx[1] + gx[2] * gx[2]);
         }
+        if (POSE) {
+            // mean: dL/dp_cam = dj^T guv;  dL/dt_c = dL/dp_cam,  dL/dW += dL/dp_cam (x) xyz
+            // covariance (J held fixed): Sigma' = J W Sigma W^T J^T  ->  dL/dW += 2 J^T G U Sigma,  Sigma = R diag(es^2) R^T
+            pose_obj = ob;
+#pragma unroll
+            for (int r = 0; r < 3; ++r) pv[r] = a0.x * dj[r] + a0.y * dj[3 + r];
+            float B0[3], B1[3];  // (G U Sigma) rows
+            {
+                float A0[3], A1[3];  // (G U R diag(es^2)) rows
+#pragma unroll
+                for (int j = 0; j < 3; ++j) {
+                    float u0 = 0.0f, u1 = 0.0f;
+#pragma unroll
+                    for (int l = 0; l < 3; ++l) {
+                        u0 += (g00 * U[l] + g01 * U[3 + l]) * R[l * 3 + j];
+                        u1 += (g01 * U[l] + g11 * U[3 + l]) * R[l * 3 + j];
+                    }
+                    const float e2 = es[j] * es[j];
+                    A0[j] = u0 * e2;
+                    A1[j] = u1 * e2;
+                }
+#pragma unroll
+                for (int c = 0; c < 3; ++c) {
+                    B0[c] = A0[0] * R[c * 3] + A0[1] * R[c * 3 + 1] + A0[2] * R[c * 3 + 2];
+                    B1[c] = A1[0] * R[c * 3] + A1[1] * R[c * 3 + 1] + A1[2] * R[c * 3 + 2];
+                }
+            }
+            const float xv[3] = {x, y, z};
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                pv[3 + c] = pv[0] * xv[c] + 2.0f * (J[0] * B0[c]);
+                pv[6 + c] = pv[1] * xv[c] + 2.0f * (J[4] * B1[c]);
+                pv[9 + c] = pv[2] * xv[c] + 2.0f * (J[2] * B0[c] + J[5] * B1[c]);
+            }
+        }
         if (COMPACT) {
             float4 *gc = reinterpret_cast<float4 *>(my_feat);
             gc[0] = make_float4(gx[0], gx[1], gx[2], gq[0] * p.q_f);
@@ -527,6 +620,22 @@ backward_points_kernel(const PointsBwdParams p) {
                 gf[2 + 4 * ch + k4] = make_float4(o16[4 * k4], o16[4 * k4 + 1], o16[4 * k4 + 2], o16[4 * k4 + 3]);
         }
         }
+      }
+      if (POSE) {
+          // one fold per object present in the warp's 32 rows, lowest lane's object first
+          const unsigned int group = __match_any_sync(0xffffffffu, pose_obj);
+          unsigned int todo = __ballot_sync(0xffffffffu, pose_obj >= 0);
+          while (todo) {
+              const int leader = __ffs(todo) - 1;
+              const int obj = __shfl_sync(0xffffffffu, pose_obj, leader);
+              todo &= ~__shfl_sync(0xffffffffu, group, leader);
+              const bool mine = pose_obj == obj;
+              float v[12];
+#pragma unroll
+              for (int k = 0; k < 12; ++k) v[k] = mine ? pv[k] : 0.0f;
+              warp_transpose_reduce12(v, lane);
+              if (reduce12_writer(lane)) s_pose[warp][obj][reduce12_slot(lane)] += v[0];
+          }
       }
       __syncwarp();
       const long long rows = p.N - base < 32 ? p.N - base : 32;
@@ -561,6 +670,86 @@ backward_points_kernel(const PointsBwdParams p) {
       }
       __syncwarp();
     }
+    if (POSE) {  // the CTA's sums, warps added in warp order
+        __syncthreads();
+        for (int k = threadIdx.x; k < p.pose_num_objects * 12; k += blockDim.x) {
+            float acc = s_pose[0][k / 12][k % 12];
+#pragma unroll
+            for (int w = 1; w < GSB_POINTS_THREADS / 32; ++w) acc += s_pose[w][k / 12][k % 12];
+            p.pose_partials[(size_t)blockIdx.x * p.pose_num_objects * 12 + k] = acc;
+        }
+    }
+}
+
+// d/d(x,y,z,w) of sum_ab G_ab R_ab for the rotation polynomial R(x,y,z,w) of GP3D:30-48 (no normalisation)
+__device__ __forceinline__ void rotation_polynomial_vjp(float x, float y, float z, float w, const float (&G)[9], float (&g)[4]) {
+    g[0] = 2 * y * G[1] + 2 * z * G[2] + 2 * y * G[3] - 4 * x * G[4] - 2 * w * G[5] + 2 * z * G[6] + 2 * w * G[7] - 4 * x * G[8];
+    g[1] = -4 * y * G[0] + 2 * x * G[1] + 2 * w * G[2] + 2 * x * G[3] + 2 * z * G[5] - 2 * w * G[6] + 2 * z * G[7] - 4 * y * G[8];
+    g[2] = -4 * z * G[0] - 2 * w * G[1] + 2 * x * G[2] + 2 * w * G[3] - 4 * z * G[4] + 2 * y * G[5] + 2 * x * G[6] + 2 * y * G[7];
+    g[3] = -2 * z * G[1] + 2 * y * G[2] + 2 * z * G[3] - 2 * x * G[5] - 2 * y * G[6] + 2 * x * G[7];
+}
+
+// One CTA per object: adds the per-CTA partials of backward_points_kernel<*, true> (each thread a fixed, strided set of
+// blocks in block order, then a fixed tree over the threads) and takes (dL/dW, dL/dt_c) to (dL/dq, dL/dt) through what
+// pose_kernel (preprocess.cu) computes from q_pointcloud_camera, t_pointcloud_camera:
+//   qi = conj(q),  W = R(qi) (polynomial, qi NOT normalised),  t_c = -R(qi / |qi|) t.
+constexpr int POSE_FINALIZE_THREADS = 128;
+__global__ void __launch_bounds__(POSE_FINALIZE_THREADS)
+pose_grad_finalize_kernel(const float *partials, int num_blocks, int n_obj, const float *q_pc, const float *t_pc,
+                          float *grad_q, float *grad_t) {
+    __shared__ float s_sum[12][POSE_FINALIZE_THREADS];
+    const int obj = blockIdx.x, tid = threadIdx.x;
+    float acc[12];
+#pragma unroll
+    for (int k = 0; k < 12; ++k) acc[k] = 0.0f;
+    for (int b = tid; b < num_blocks; b += POSE_FINALIZE_THREADS) {
+        const float *row = partials + ((size_t)b * n_obj + obj) * 12;
+#pragma unroll
+        for (int k = 0; k < 12; ++k) acc[k] += row[k];
+    }
+#pragma unroll
+    for (int k = 0; k < 12; ++k) s_sum[k][tid] = acc[k];
+    for (int h = POSE_FINALIZE_THREADS / 2; h > 0; h >>= 1) {
+        __syncthreads();
+        if (tid < h) {
+#pragma unroll
+            for (int k = 0; k < 12; ++k) s_sum[k][tid] += s_sum[k][tid + h];
+        }
+    }
+    __syncthreads();
+    if (tid != 0) return;
+    const float gtc[3] = {s_sum[0][0], s_sum[1][0], s_sum[2][0]};
+    float gW[9];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) gW[k] = s_sum[3 + k][0];
+    const float qi[4] = {-q_pc[4 * obj], -q_pc[4 * obj + 1], -q_pc[4 * obj + 2], q_pc[4 * obj + 3]};
+    const float t[3] = {t_pc[3 * obj], t_pc[3 * obj + 1], t_pc[3 * obj + 2]};
+    const float n = sqrtf(qi[0] * qi[0] + qi[1] * qi[1] + qi[2] * qi[2] + qi[3] * qi[3]);
+    const float qn[4] = {qi[0] / n, qi[1] / n, qi[2] / n, qi[3] / n};
+    const float x = qn[0], y = qn[1], z = qn[2], w = qn[3];
+    const float Rn[9] = {1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y),
+                         2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x),
+                         2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)};
+    // t_c = -Rn t:  dL/dt = -Rn^T dL/dt_c,  dL/dRn = -dL/dt_c (x) t
+#pragma unroll
+    for (int c = 0; c < 3; ++c) grad_t[3 * obj + c] = -(Rn[c] * gtc[0] + Rn[3 + c] * gtc[1] + Rn[6 + c] * gtc[2]);
+    float gRn[9];
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = 0; b < 3; ++b) gRn[a * 3 + b] = -gtc[a] * t[b];
+    float gqn[4], gqi[4];
+    rotation_polynomial_vjp(x, y, z, w, gRn, gqn);
+    rotation_polynomial_vjp(qi[0], qi[1], qi[2], qi[3], gW, gqi);
+    // qn = qi / |qi|:  dL/dqi += (dL/dqn - qn (qn . dL/dqn)) / |qi|
+    const float dot = qn[0] * gqn[0] + qn[1] * gqn[1] + qn[2] * gqn[2] + qn[3] * gqn[3];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) gqi[k] += (gqn[k] - qn[k] * dot) / n;
+    // qi = conj(q)
+    grad_q[4 * obj] = -gqi[0];
+    grad_q[4 * obj + 1] = -gqi[1];
+    grad_q[4 * obj + 2] = -gqi[2];
+    grad_q[4 * obj + 3] = gqi[3];
 }
 
 // ------------------------------------------------------------------ view-parallel exchange: rebuild the dense gradients
@@ -661,8 +850,17 @@ expand_view_gradients_kernel(const ExpandParams p) {
 #ifndef GSB_HOST_EMU
 static int first_cleared_of_band(int band) { return band <= 0 ? 1 : band == 1 ? 4 : band == 2 ? 9 : 16; }
 
-int launch_backward_points(const GsbBackwardArgs &a, const Workspace &ws, cudaStream_t stream, const long long *skip_flag) {
-    if (a.num_points <= 0) return GSB_OK;
+int launch_backward_points(const GsbBackwardArgs &a, const Workspace &ws, cudaStream_t stream, const long long *skip_flag,
+                           const GsbPoseGradArgs *pose) {
+    if (a.num_points <= 0) {
+        if (pose) {  // no rows: every object gets zeros
+            pose_grad_finalize_kernel<<<a.num_objects, POSE_FINALIZE_THREADS, 0, stream>>>(
+                static_cast<const float *>(pose->temp), 0, a.num_objects, pose->q_pointcloud_camera,
+                pose->t_pointcloud_camera, pose->grad_q_pointcloud_camera, pose->grad_t_pointcloud_camera);
+            GSB_CUDA_CHECK(cudaGetLastError());
+        }
+        return GSB_OK;
+    }
     PointsBwdParams p;
     p.ctl_num_in_camera = a.ctl_accumulated_num_in_camera;
     p.ctl_num_pixels = a.ctl_accumulated_num_pixels;
@@ -692,12 +890,26 @@ int launch_backward_points(const GsbBackwardArgs &a, const Workspace &ws, cudaSt
     p.grad_feat = a.grad_pointcloud_features;
     p.grad_sum_compact = a.grad_sum_compact;
     p.grad_color_compact = a.grad_color_compact;
+    p.pose_num_objects = pose ? a.num_objects : 0;
+    p.pose_partials = pose ? static_cast<float *>(pose->temp) : nullptr;
     long long blocks = (a.num_points + GSB_POINTS_THREADS - 1) / GSB_POINTS_THREADS;
     const long long cap = 16LL * num_sms();
     if (blocks > cap) blocks = cap;
+    if (pose && blocks > POSE_MAX_BLOCKS) blocks = POSE_MAX_BLOCKS;  // the partials of gsb200_pose_grad_temp_bytes
     if (blocks <= 0) return GSB_OK;
-    if (a.flags & GSB_FLAG_COMPACT_GRADS) backward_points_kernel<true><<<(int)blocks, GSB_POINTS_THREADS, 0, stream>>>(p);
-    else backward_points_kernel<false><<<(int)blocks, GSB_POINTS_THREADS, 0, stream>>>(p);
+    const bool compact = (a.flags & GSB_FLAG_COMPACT_GRADS) != 0;
+    if (pose) {
+        if (compact) backward_points_kernel<true, true><<<(int)blocks, GSB_POINTS_THREADS, 0, stream>>>(p);
+        else backward_points_kernel<false, true><<<(int)blocks, GSB_POINTS_THREADS, 0, stream>>>(p);
+        GSB_CUDA_CHECK(cudaGetLastError());
+        pose_grad_finalize_kernel<<<a.num_objects, POSE_FINALIZE_THREADS, 0, stream>>>(
+            p.pose_partials, (int)blocks, a.num_objects, pose->q_pointcloud_camera, pose->t_pointcloud_camera,
+            pose->grad_q_pointcloud_camera, pose->grad_t_pointcloud_camera);
+    } else if (compact) {
+        backward_points_kernel<true><<<(int)blocks, GSB_POINTS_THREADS, 0, stream>>>(p);
+    } else {
+        backward_points_kernel<false><<<(int)blocks, GSB_POINTS_THREADS, 0, stream>>>(p);
+    }
     GSB_CUDA_CHECK(cudaGetLastError());
     return GSB_OK;
 }

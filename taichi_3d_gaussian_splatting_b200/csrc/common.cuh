@@ -25,6 +25,9 @@ void set_error(const char *fmt, ...);
 // CNT_MAX_DEPTH_KEY: largest int32(depth * scale) over the frame's in-camera points (low 32 bits of the slot; the per-point
 // kernel atomicMax-es it, the sort derives the number of live depth bits from it)
 enum Counter { CNT_M = 0, CNT_K = 1, CNT_OVERFLOW = 2, CNT_MAX_DEPTH_KEY = 4 };
+// gsb200_backward_with_pose: the per-point kernel runs on at most this many CTAs, so that its per-CTA pose partials fit the
+// temp size gsb200_pose_grad_temp_bytes gives without asking the device (16 CTAs per SM up to 256 SMs)
+constexpr int POSE_MAX_BLOCKS = 4096;
 enum Ticket { TICKET_SCAN = 0, TICKET_SORT0 = 1 /* ..+7: one per pass; +8: histogram blocks done */ };
 
 // Per-object pose block in the workspace (20 floats):
@@ -71,8 +74,9 @@ int launch_tile_ranges_raw(const long long *keys_i64, int64_t n, int *tile_start
                            int num_tiles, cudaStream_t stream);
 int launch_blend_forward(const GsbForwardArgs &a, const Workspace &ws, cudaStream_t stream);
 int launch_blend_backward(const GsbBackwardArgs &a, const Workspace &ws, cudaStream_t stream);
+// pose: gsb200_backward_with_pose's outputs (the POSE instantiation of the per-point kernel + its finalisation), or nullptr
 int launch_backward_points(const GsbBackwardArgs &a, const Workspace &ws, cudaStream_t stream,
-                           const long long *skip_flag = nullptr);
+                           const long long *skip_flag = nullptr, const GsbPoseGradArgs *pose = nullptr);
 int launch_adam_step(float *param, const float *grad, float *exp_avg, float *exp_avg_sq, long long n, double lr, double beta1,
                      double beta2, double eps, int step, const long long *skip_flag, cudaStream_t stream);
 int launch_expand_view_gradients(const GsbExpandArgs &a, cudaStream_t stream);
